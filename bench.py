@@ -14,6 +14,10 @@ Y (fill) and Z (extend) — six fused ``xg_stencil2`` launches, 6 x 648 M output
   cpu_baseline  the oracle (numpy restatement of the reference's calls: np.pad + ufunc on a
           moveaxis view) timed single-threaded on the host, rank 0, N=1, on a bounded sample.
 
+``--dump-outputs DIR`` writes what the last timed step returned, one ``DIR/<op>_<axis>.npy`` (fp32) per Grid call:
+a seeded sub-block (DUMP_SAMPLE levels x rows x columns, both edges of every axis included) of each output, the
+same cells on every run with the same arguments, so two builds can be compared output for output.
+
 ``--impl reference`` times the reference's own CPU path (the oracle port; xarray/dask are not
 installable, see DESIGN.md) with a thread pool over all host cores on broadcast-dim chunks —
 the dask="parallelized" analogue (xgcm/grid.py:786-789).
@@ -44,6 +48,7 @@ SEED = 0xC0FFEE
 AXES = (("X", "periodic", None), ("Y", "fill", 0.0), ("Z", "extend", None))
 OPS = ("diff", "interp")
 METRIC = "grid-cells/s for diff+interp on C-grid field; achieved HBM GB/s vs peak"
+DUMP_SAMPLE = (16, 128, 1024)  # (Z, Y, X) indices kept per output by --dump-outputs: 8 MiB fp32 each, 48 MiB for six
 WORKLOAD = ("C3 (BASELINE configs[2]): Grid.diff + Grid.interp along X(periodic), Y(fill), Z(extend) of one "
             "75x2400x3600 fp32 C-grid field per step")
 
@@ -58,7 +63,14 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the per-config records (C1, C2, C3 integrate, C4 loop, C5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of each output of the last timed step to DIR/<op>_<axis>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def measured_peak():
@@ -67,6 +79,20 @@ def measured_peak():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_sample_index(shape):
+    """Sorted indices along (Z, Y, X) for --dump-outputs: the first and last two of every axis, where the
+    boundary conditions act, plus seeded random interior ones; the whole axis when it is short."""
+    rng = np.random.default_rng(SEED)
+    idx = []
+    for n, k in zip(shape, DUMP_SAMPLE):
+        if n <= k:
+            idx.append(np.arange(n))
+        else:
+            inner = rng.choice(np.arange(2, n - 2), k - 4, replace=False)
+            idx.append(np.sort(np.concatenate([[0, 1, n - 2, n - 1], inner])))
+    return idx
 
 
 def make_dataset(shape, field):
@@ -500,8 +526,13 @@ def run_ours(args):
     x = torch.empty(shape, dtype=torch.float32, device=dev)
     ops.fill_uniform(x, SEED, offset=rank * cells_field)
     grid, da_dev = make_dataset(shape, x)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        iz, iy, ix = (torch.as_tensor(i, device=dev) for i in dump_sample_index(shape))
+        sample_at = (iz[:, None, None], iy[None, :, None], ix[None, None, :])
+        dumped = {}
 
-    def step_device(timer=None):
+    def step_device(timer=None, keep=None):
         n = 0
         for ax, bc, fill in AXES:
             for op in OPS:
@@ -511,6 +542,8 @@ def run_ours(args):
                 r = getattr(grid, op)(da_dev, ax)
                 if timer is not None:
                     timer[-1][3].record()
+                if keep is not None:
+                    keep[f"{op}_{ax}"] = r
                 n += r.size
                 del r
         return n
@@ -522,8 +555,10 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     # ---- value: inputs resident in HBM ------------------------------------------------------
-    for _ in range(max(args.warmup, 3)):
-        step_device()
+    for i in range(max(args.warmup, 3)):
+        # a warm-up step that keeps its results leaves their memory in the allocator's cache, so keeping the
+        # last timed step's results for --dump-outputs allocates nothing inside the timed window
+        step_device(keep={} if dumped is not None and i == 0 else None)
     barrier()
     sampler = ClockSampler(torch.cuda.current_device())
     if rank == 0:
@@ -534,10 +569,15 @@ def run_ours(args):
     barrier()
     e0.record()
     cells = 0
-    for _ in range(args.steps):
-        cells += step_device(timers)
+    for i in range(args.steps):
+        cells += step_device(timers, dumped if i == args.steps - 1 else None)
     e1.record()
     barrier()
+    if dumped:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, r in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), r.data[sample_at].cpu().numpy())
+        dumped.clear()
     launches = lib.xg_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)

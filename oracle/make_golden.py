@@ -1,8 +1,8 @@
 """Generate tests/golden/* by RUNNING the reference's unmodified kernels.
 
-Run in the build container only (needs /root/reference):
+Needs a source checkout of xgcm (the committed vectors come from xgcm 052b033a):
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden PATH_TO_XGCM_CHECKOUT
 
 Outputs (small, committed):
   tests/golden/gridops_ref.npz      every <op>_<from>_to_<to> GridUFunc of xgcm/gridops.py applied to
@@ -14,6 +14,9 @@ Outputs (small, committed):
                                     decreasing / kinked columns, decreasing bins
   tests/golden/transform_cases.json the linear / log / conservative entries of the `cases` dict of
                                     xgcm/test/test_transform.py:41-683 (inputs + expected values)
+  tests/golden/live_kernels_ref.npz every diff / interp / min / max GridUFunc on a periodic-padded fp64
+                                    field along each axis, and interp_1d_linear on columns (every third
+                                    one decreasing), with and without mask_edges
 
 TEST INFRASTRUCTURE ONLY.
 """
@@ -22,6 +25,7 @@ from __future__ import annotations
 
 import json
 import re
+import sys
 from pathlib import Path
 
 import numpy as np
@@ -123,8 +127,33 @@ def conservative_vectors(transform):
     return out
 
 
-def transform_cases():
-    src = (ref_loader.REFERENCE_ROOT / "xgcm" / "test" / "test_transform.py").read_text()
+def live_kernel_vectors(gridops, transform):
+    rng = np.random.default_rng(0)
+    a = rng.random((3, 4, 7))
+    out = {"a": a}
+    names = [n for n in dir(gridops) if re.match(r"^(diff|interp|min|max)_\w+_to_\w+$", n)]
+    for name in sorted(names):
+        gu = getattr(gridops, name)
+        if gu.padding_width is None:
+            continue
+        lo, hi = gu.padding_width["X"]
+        for axis in range(3):
+            widths = [(0, 0)] * 3
+            widths[axis] = (lo, hi)
+            p = np.pad(a, widths, mode="wrap")
+            out[f"{name}|{axis}"] = np.moveaxis(gu.ufunc(np.moveaxis(p, axis, -1)), -1, axis)
+    phi = rng.random((40, 30))
+    theta = np.cumsum(rng.random((40, 30)) + 0.1, axis=-1)
+    theta[::3] = theta[::3, ::-1]
+    target = np.linspace(-1, theta.max() + 1, 25)
+    out.update({"phi": phi, "theta": theta, "target": target})
+    for mask in (False, True):
+        out[f"interp_1d_linear|{int(mask)}"] = transform.interp_1d_linear(phi, theta, target, mask_edges=mask)
+    return out
+
+
+def transform_cases(root):
+    src = (Path(root) / "xgcm" / "test" / "test_transform.py").read_text()
     start = src.index("cases = {")
     end = src.index("def construct_test_source_data")
     ns = {"np": np}
@@ -154,14 +183,18 @@ def transform_cases():
 
 
 def main():
-    gridops, transform = ref_loader.load()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python -m oracle.make_golden PATH_TO_XGCM_CHECKOUT")
+    root = sys.argv[1]
+    gridops, transform = ref_loader.load(root)
     GOLDEN.mkdir(parents=True, exist_ok=True)
     vec, table = gridops_vectors(gridops)
     np.savez_compressed(GOLDEN / "gridops_ref.npz", **vec)
     (GOLDEN / "gridops_table.json").write_text(json.dumps(table, indent=1, sort_keys=True))
     np.savez_compressed(GOLDEN / "interp1d_ref.npz", **interp1d_vectors(transform))
     np.savez_compressed(GOLDEN / "conservative_ref.npz", **conservative_vectors(transform))
-    (GOLDEN / "transform_cases.json").write_text(json.dumps(transform_cases(), indent=1, sort_keys=True))
+    (GOLDEN / "transform_cases.json").write_text(json.dumps(transform_cases(root), indent=1, sort_keys=True))
+    np.savez_compressed(GOLDEN / "live_kernels_ref.npz", **live_kernel_vectors(gridops, transform))
     for p in sorted(GOLDEN.iterdir()):
         print(p.name, p.stat().st_size)
 

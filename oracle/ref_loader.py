@@ -1,11 +1,10 @@
-"""Import the reference's UNMODIFIED kernels from /root/reference (this container only).
+"""Import the reference's UNMODIFIED kernels from an xgcm source checkout.
 
-xarray and dask are not installed and cannot be installed here, so ``import xgcm``
-fails; but ``xgcm.gridops`` and ``xgcm.transform`` only need those packages for
-def-time type annotations.  We register empty stand-in modules exposing the
-referenced type names and import the two kernel modules as they lie on disk.
-Nothing is copied.  Used by ``oracle/make_golden.py`` and by the (auto-skipped
-when the tree is absent) cross-check in ``tests/test_oracle_golden.py``.
+xarray and dask need not be installed: ``xgcm.gridops`` and ``xgcm.transform``
+only need those packages for def-time type annotations.  We register empty
+stand-in modules exposing the referenced type names and import the two kernel
+modules as they lie on disk.  Nothing is copied.  Used by ``oracle/make_golden.py``
+to record the golden vectors under ``tests/golden/``.
 
 TEST INFRASTRUCTURE ONLY.
 """
@@ -17,12 +16,6 @@ import sys
 import types
 from pathlib import Path
 
-REFERENCE_ROOT = Path("/root/reference")
-
-
-def available() -> bool:
-    return (REFERENCE_ROOT / "xgcm" / "gridops.py").exists()
-
 
 def _stub(name: str, **attrs):
     mod = types.ModuleType(name)
@@ -31,10 +24,11 @@ def _stub(name: str, **attrs):
     return mod
 
 
-def load():
-    """Return ``(gridops, transform)`` modules of the reference."""
-    if not available():
-        raise RuntimeError("/root/reference is not present on this machine")
+def load(root):
+    """Return ``(gridops, transform)`` modules of the reference checkout at ``root``."""
+    root = Path(root)
+    if not (root / "xgcm" / "gridops.py").is_file():
+        raise RuntimeError(f"{root} is not an xgcm source checkout (no xgcm/gridops.py)")
     added = []
     if "xarray" not in sys.modules:
         sys.modules["xarray"] = _stub(
@@ -50,7 +44,7 @@ def load():
         added += ["dask", "dask.array"]
     # import xgcm's submodules without running xgcm/__init__.py (which needs xarray for real)
     pkg = types.ModuleType("xgcm")
-    pkg.__path__ = [str(REFERENCE_ROOT / "xgcm")]
+    pkg.__path__ = [str(root / "xgcm")]
     prev = sys.modules.get("xgcm")
     sys.modules["xgcm"] = pkg
     try:
