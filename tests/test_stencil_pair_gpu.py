@@ -107,7 +107,7 @@ def test_pair_argument_validation():
 
 def test_divergence_full_size_samples():
     """C3-sized divergence: sampled blocks against the chain."""
-    from xgcm_b200 import ops
+    from xgcm_b200 import _capi, ops
 
     nz, ny, nx = 75, 2400, 3600
     u = torch.empty((nz, ny, nx), dtype=torch.float32, device=DEV)
@@ -120,6 +120,7 @@ def test_divergence_full_size_samples():
     ra = (dx * dy).astype(np.float32)
     out = ops.stencil_pair(u, v, ("diff", 0, 1, "periodic", 0.0), (1, "diff", 0, 1, "periodic", 0.0), 0,
                            pre_a=_t(dy), pre_b=_t(dx), post=_t(ra))
+    assert _capi.last_launch() == "xg_stencil_pair(tile_tma)"
     rng = np.random.default_rng(5)
     for _ in range(4):
         k = int(rng.integers(0, nz))

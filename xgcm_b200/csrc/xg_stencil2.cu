@@ -646,6 +646,9 @@ __global__ void __launch_bounds__(kTmaConsumers + 32, 3)
       if (edge_lane) pnb = ps[NBI];
     }
     const int64_t row0 = (int64_t)z0 * a.P + prow;
+    // the spare rows of the last tile row (prow >= P, nothing stored) load their global operands at the last row:
+    // unclamped they would run past the field's, the halo's and the pre-metric's last level
+    const int prc = prow < a.P ? prow : (int)a.P - 1;
     const bool at_edge = LO ? (x == 0) : (x + VEC >= a.n);
     T* op = a.out + row0 * a.n + x;
 #pragma unroll
@@ -660,7 +663,7 @@ __global__ void __launch_bounds__(kTmaConsumers + 32, 3)
           *reinterpret_cast<V*>(pv.v) = *reinterpret_cast<const V*>(ps + u * LS);
           if (edge_lane) pnb = ps[u * LS + NBI];
         } else if (pre_scalar) {
-          pnb = __ldg(prep + xg_groups_offset(a.pre.outer, row0 + u * a.P));
+          pnb = __ldg(prep + xg_groups_offset(a.pre.outer, (int64_t)(z0 + u) * a.P + prc));
 #pragma unroll
           for (int kk = 0; kk < VEC; ++kk) pv.v[kk] = pnb;
         }
@@ -672,7 +675,7 @@ __global__ void __launch_bounds__(kTmaConsumers + 32, 3)
       if (edge_lane) nb = enb;
       if (at_edge) {
         // A[row, s] = in * pre straight from global memory: the row's other end (periodic) only
-        const int64_t row = row0 + u * a.P;
+        const int64_t row = (int64_t)(z0 + u) * a.P + prc;
         auto A = [&](int64_t s_) -> T {
           T val = __ldg(a.in + row * a.n + s_);
           if (PRE != XG_PRE_NONE) val = val * __ldg(prep + xg_groups_offset(a.pre.outer, row) + s_ * a.pre.axis_stride);

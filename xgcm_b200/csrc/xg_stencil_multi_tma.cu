@@ -193,6 +193,9 @@ __global__ void __launch_bounds__(kConsumersM + 32, 3)
         if (lz < lvls)
           for (int c = tid; c < rows_box * BOXW; c += kConsumersM) fix(lz, c / BOXW, c % BOXW);
       }
+      // the cells above are generic-proxy writes into a stage the producer later refills through the async
+      // proxy (cp.async.bulk.tensor): order them before this thread's share of the empty-barrier arrive
+      fence_async_smem();
       asm volatile("bar.sync 1, %0;" ::"r"(kConsumersM) : "memory");
     }
 

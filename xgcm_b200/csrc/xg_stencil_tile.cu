@@ -276,18 +276,20 @@ __global__ void __launch_bounds__(kConsumers + 32, HAS_A ? 2 : 3)  // the pair's
         b1.v[kk] = b1.v[kk] * mb1.v[kk];
       }
       if (low_b || high_b) {
-        // (B x mb)[z, row, x .. x + VEC) from global memory: wrap-around and extrapolation partners
+        // (B x mb)[z, row, x .. x + VEC) from global memory: wrap-around and extrapolation partners.  The spare
+        // lanes of the last, partial x tile (x >= n, nothing stored) load at the row's last vector instead
+        const int xl = x < n ? x : (int)n - VEC;
         auto Brow = [&](int64_t row) -> Pack {
-          Pack r = xg_ld_cached<T, VEC>(s.b + z * bsz + row * fsp + x);
+          Pack r = xg_ld_cached<T, VEC>(s.b + z * bsz + row * fsp + xl);
           if (mb_mode != M_NONE) {
 #pragma unroll
             for (int kk = 0; kk < VEC; ++kk)
-              r.v[kk] = r.v[kk] * __ldg(s.mb.ptr + z * s.mb.sz + row * s.mb.sp + (int64_t)(x + kk) * s.mb.sx);
+              r.v[kk] = r.v[kk] * __ldg(s.mb.ptr + z * s.mb.sz + row * s.mb.sp + (int64_t)(xl + kk) * s.mb.sx);
           }
           return r;
         };
         if (low_b) {  // s0 == -1
-          if (s.halo_lo) b0 = xg_ld_cached<T, VEC>(s.halo_lo + z * n + x);
+          if (s.halo_lo) b0 = xg_ld_cached<T, VEC>(s.halo_lo + z * n + xl);
           else if (s.bc_b == XG_BC_FILL) {
 #pragma unroll
             for (int kk = 0; kk < VEC; ++kk) b0.v[kk] = s.fill_b;
@@ -300,7 +302,7 @@ __global__ void __launch_bounds__(kConsumers + 32, HAS_A ? 2 : 3)  // the pair's
           }
         }
         if (high_b) {  // s1 == Pb
-          if (s.halo_hi) b1 = xg_ld_cached<T, VEC>(s.halo_hi + z * n + x);
+          if (s.halo_hi) b1 = xg_ld_cached<T, VEC>(s.halo_hi + z * n + xl);
           else if (s.bc_b == XG_BC_FILL) {
 #pragma unroll
             for (int kk = 0; kk < VEC; ++kk) b1.v[kk] = s.fill_b;
